@@ -20,6 +20,8 @@ rank, so the per-GPU work is the same at every N: weak scaling).
   configs2 / mode_F   extra keys: configs[2] (128-beam, 0.05 m grid, correlative + refine) and the full-cloud matcher mode.
 
 `--impl reference` times the CPU chain alone (all host threads) and prints the same line with "impl": "reference".
+`--dump-outputs DIR` writes what the last timed step returned (rank 0) as float64 .npy files, see dump_outputs(); the inputs are
+seeded, so two builds run with the same arguments can be compared output for output.
 Inputs per step exceed L2 (148 scans x 2.1 MB = 309 MB > 126 MB), so no explicit L2 flush.
 """
 import argparse
@@ -37,6 +39,7 @@ import time
 if os.environ.get("NCCL_DEBUG", "").upper() == "VERSION":
     os.environ["NCCL_DEBUG"] = "WARN"
 os.environ.setdefault("NCCL_DEBUG_FILE", "/dev/stderr")
+sys.dont_write_bytecode = True   # the benchmark writes nothing into the tree it runs from (which may be read-only)
 
 import numpy as np
 
@@ -182,6 +185,35 @@ def pose_errors(a, b):
     return dt, 2 * np.arccos(d)
 
 
+def struct_rows(records, struct):
+    """(len(records), k) float64 of a ctypes struct's scalar and array fields, in declaration order; nested structs and
+    `reserved` are left out (integers up to 2^53 are exact in float64)."""
+    rows = []
+    for r in records:
+        row = []
+        for name, _ in struct._fields_:
+            v = getattr(r, name)
+            if name == "reserved" or isinstance(v, C.Structure):
+                continue
+            row.extend(v[:] if isinstance(v, C.Array) else [v])
+        rows.append(row)
+    return np.array(rows, np.float64)
+
+
+def dump_outputs(path, dliom, results, states, table):
+    """What the last timed step hands its caller, one float64 .npy per array (columns in the C struct's field order):
+    states (B, 16) p q v ba bg after the solve; scan_results (B, 25) = dl_scan_result without its solve summary;
+    solve_summary (B, 7) = dl_solve_summary; constraints (rows, 15) = the exchange step's dl_constraint_row table (not
+    written with --pairs 0)."""
+    os.makedirs(path, exist_ok=True)
+    arrays = {"states": np.asarray(states, np.float64), "scan_results": struct_rows(results, dliom.ScanResult),
+              "solve_summary": struct_rows([r.summary for r in results], dliom.SolveSummary)}
+    if table is not None:
+        arrays["constraints"] = struct_rows(table, dliom.ConstraintRow)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), a)
+
+
 class ClockSampler(threading.Thread):
     """nvidia-smi clocks / throttle reasons at 2 Hz from before the warm-up to after the last timed region (a subprocess every
     500 ms; round 1 sampled at 10 Hz, which showed up as noise in a 33 ms timed region)."""
@@ -297,7 +329,13 @@ def main():
                     help="3: x y z rows + the per-point times as runs (12 B/point); 4: TimedPointCloud rows x y z t (what AddRangeData "
                          "receives); 8: RangeMeasurement rows")
     ap.add_argument("--no-extras", action="store_true", help="skip the configs[2] / mode-F / no-IMU extra measurements")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the results of the last timed step (rank 0) to DIR/<name>.npy (see dump_outputs())")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the device path's results: use it with --impl ours")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
 
     rank = int(os.environ.get("RANK", "0"))
@@ -387,6 +425,7 @@ def main():
             self.pending = 0
             self.error = None
             self.stop = False
+            self.table = None   # the constraint table of this worker's latest exchange
             self.start()
 
         def run(self):
@@ -398,6 +437,7 @@ def main():
                         return
                 try:
                     table, info = self.plan()
+                    self.table = table
                     with exchange_lock:
                         exchange["ms"].append(info.collective_ms)
                         exchange["found"] = info.found_total
@@ -522,6 +562,10 @@ def main():
     launches = sum(c.launches for c in [ctx, ctx2] + xctxs) - launches0
     profile = ctx.read_profile()
     ctx.set_profiling(False)
+    if args.dump_outputs:   # read back before the later loops reuse the lanes; the last step ran on lane (steps - 1) % 2
+        c_last, out_last, st_last, _ = dev_lanes[(args.steps - 1) % 2]
+        last_step = (c_last.fetch_results(C.c_void_p(out_last.data_ptr()), B), st_last.cpu().numpy(),
+                     workers[(submitted[0] - 1) % len(workers)].table if workers else None)
     collective_ms = float(np.median(exchange["ms"])) if exchange["ms"] else None
     note("device-resident loop done")
     # ---- timed: end to end (host buffers in, results out), streaming and blocking
@@ -711,6 +755,8 @@ def main():
                 "clocks": sampler.summary()}
         line.update(extras)
         print(json.dumps(line))
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, dliom, *last_step)
     note("line printed")
     sampler.stop_flag = True
     for wk in workers:

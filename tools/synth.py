@@ -11,23 +11,33 @@ Trajectory: 10 m/s along +x with a 0.2 rad/s-amplitude yaw sinusoid; the sensor 
 import ctypes
 import os
 import subprocess
+import tempfile
 
 import numpy as np
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
+RAYCAST_LIB = os.path.join(_HERE, "libraycast.so")
 _RAYCAST = None
 
 
+def build_raycast(path=RAYCAST_LIB):
+    """Compiles raycast.c into `path` (__graft_entry__.build() makes tools/libraycast.so)."""
+    subprocess.check_call(["gcc", "-O2", "-fopenmp", "-shared", "-fPIC", "-o", path, os.path.join(_HERE, "raycast.c"), "-lm"])
+
+
 def _raycast_lib():
-    """tools/libraycast.so (C, OpenMP): ~40x faster than the numpy path; built on first use, optional."""
+    """tools/libraycast.so (C, OpenMP): ~40x faster than the numpy path, optional. In a tree that was not built it is compiled
+    into a temporary directory, never into the tree (which may be read-only)."""
     global _RAYCAST
     if _RAYCAST is None:
-        path = os.path.join(_HERE, "libraycast.so")
         try:
-            if not os.path.exists(path):
-                subprocess.check_call(["gcc", "-O2", "-fopenmp", "-shared", "-fPIC", "-o", path,
-                                       os.path.join(_HERE, "raycast.c"), "-lm"])
-            L = ctypes.CDLL(path)
+            if os.path.exists(RAYCAST_LIB):
+                L = ctypes.CDLL(RAYCAST_LIB)
+            else:
+                with tempfile.TemporaryDirectory() as d:
+                    path = os.path.join(d, "libraycast.so")
+                    build_raycast(path)
+                    L = ctypes.CDLL(path)   # stays mapped after the directory is removed
             dp = np.ctypeslib.ndpointer(np.float64, flags="C_CONTIGUOUS")
             L.synth_raycast.argtypes = [ctypes.c_int64, dp, dp, ctypes.c_double, ctypes.c_double, ctypes.c_int, dp, dp,
                                         ctypes.c_int, dp, ctypes.c_double, ctypes.c_double, dp]
